@@ -14,7 +14,7 @@ Extra legs in the same JSON line (all device-timed with CUDA events unless state
   pipeline_e2e              BASELINE configs[4]'s per-GPU work: pipeline.MfDetectPipeline, int32 counts up, picks down
   cpu_baseline              the oracle port of the reference path on the box's host cores (N=1 only)
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -38,6 +38,7 @@ METRIC = "DAS channels/sec through f-k filter"
 WORKLOAD = f"synthetic {NX} ch x {NS} samp fp32, f-k filter only (fk_filter_design fan mask {FAN}), one matrix per GPU"
 CONFIG = {"workload": WORKLOAD, "l2": "inputs (4.8 GB) exceed the 126 MB L2; no flush needed"}   # identical in both arms
 CPU_SAMPLE_NX = 250                 # single-thread sample: 250 channels x the full 120 000 samples
+DUMP_ROWS, DUMP_SEED = 128, 0       # --dump-outputs: 128 full channels of the 4.8 GB output = 61 MB of float32
 SHARD_NX, SHARD_NS = 20000, 240000  # BASELINE configs[3]
 
 # ncu --set full dram__bytes_read.sum + dram__bytes_write.sum per launch, keyed by what was profiled: (column scheme,
@@ -240,6 +241,10 @@ def main():
     ap.add_argument("--no-hybrid", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the filtered matrix of the last step as DIR/fk_filter_filt.npy: "
+                         f"float32, the {DUMP_ROWS} channels drawn by numpy.random.default_rng({DUMP_SEED}), in ascending order "
+                         "(rank 0's matrix when --gpus > 1)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -323,6 +328,10 @@ def main():
     e1.record()
     barrier()
     launches = L.d4w_launch_count() - n0
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump_rows = np.sort(np.random.default_rng(DUMP_SEED).choice(NX, size=DUMP_ROWS, replace=False))
+        dump = y[torch.from_numpy(dump_rows).to(y.device)].cpu().numpy()
     clocks = None
     if rank == 0:
         # nvidia-smi reports every 100 ms; a short timed region (K steps of ~8 ms) may see fewer than three reports, so
@@ -615,6 +624,9 @@ def main():
                                     "single_thread": {"value": sv, "unit": "channels/s", "cores": 1,
                                                       "kind": reference_source(),
                                                       "sample": f"{CPU_SAMPLE_NX} ch x {NS} samp ({st:.1f} s), numpy.fft as the reference calls it"}}
+        if dump is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "fk_filter_filt.npy"), dump)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -203,6 +203,7 @@ def main():
     np.savez_compressed(os.path.join(OUT, "raw2strain.npz"), raw=raw, scale_factor=meta["scale_factor"], strain=ref_strain)
 
     rep.update(make_round2())
+    rep.update(make_spot())
     for k, v in rep.items():
         print(f"{k:24s} oracle-vs-reference rel err {v:.2e}")
     tot = sum(os.path.getsize(os.path.join(OUT, f)) for f in os.listdir(OUT))
@@ -287,9 +288,46 @@ def make_round2():
     return rep
 
 
+def make_spot():
+    """Reference outputs on the seeded white-noise inputs of the spot checks in tests/test_oracle_golden.py (spot.npz).
+    Every third row of the larger 2-D outputs is stored, which keeps the file small."""
+    from oracle import improcess_oracle as IO
+    dsp, detect = ref_loader.load()
+    imp = ref_loader.load_improcess()
+    rep = {}
+    sp = {}
+    nx, ns = 36, 200
+    x = np.random.default_rng(5).standard_normal((nx, ns))
+    sel = [0, nx, 1]
+    m = dsp.fk_filter_design((nx, ns), sel, DX, FS)
+    assert np.array_equal(m, O.fk_filter_design((nx, ns), sel, DX, FS))
+    y = dsp.fk_filter_filt(x.copy(), m, True)
+    rep["spot_fk"] = close(y, O.fk_filter_filt(x.copy(), m, True), tol=1e-13, what="fk_filter_filt")
+    h = np.asarray(dsp.hybrid_ninf_filter_design((nx, ns), sel, DX, FS))
+    rep["spot_ninf"] = close(h, O.hybrid_ninf_filter_design((nx, ns), sel, DX, FS), tol=1e-13, what="hybrid_ninf")
+    bp = dsp.bp_filt(x, FS, 14, 30)
+    rep["spot_bp"] = close(bp, O.bp_filt(x, FS, 14, 30), tol=1e-13, what="bp_filt")
+    tpl = detect.gen_template_fincall(np.arange(ns) / FS, FS, 17.8, 28.8, 0.68)
+    xc = detect.compute_cross_correlogram(x, tpl)
+    rep["spot_xc"] = close(xc, D.compute_cross_correlogram(x, tpl), tol=1e-13, what="cross_correlogram")
+    sp.update(a_x_checksum=float(np.sum(x)), a_mask=m, a_ninf=h, a_tpl=tpl, a_fk_rows=y[::3], a_bp_rows=bp[::3], a_xc_rows=xc[::3])
+    x = np.random.default_rng(8).standard_normal((30, 500))
+    fx = dsp.get_fx(x, 256)
+    rep["spot_get_fx"] = close(fx, O.get_fx(x, 256), tol=1e-14, what="get_fx")
+    img = imp.trace2image(x)
+    rep["spot_trace2image"] = close(img, IO.trace2image(x), tol=1e-13, what="trace2image")
+    b = imp.binning(img, 0.1, 0.1)
+    rep["spot_binning"] = close(b, IO.binning(img, 0.1, 0.1), tol=1e-13, what="binning")
+    up, down = imp.gabor_filt_design(40.0)
+    assert np.array_equal(up, IO.gabor_filt_design(40.0)[0]) and np.array_equal(down, np.flipud(up))
+    sp.update(b_x_checksum=float(np.sum(x)), b_fx_rows=fx[::3], b_img_rows=img[::3], b_bin=b, b_up=up)
+    np.savez_compressed(os.path.join(OUT, "spot.npz"), **sp)
+    return rep
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "round2":
-        for k, v in make_round2().items():
+    if len(sys.argv) > 1 and sys.argv[1] in ("round2", "spot"):
+        for k, v in (make_round2() if sys.argv[1] == "round2" else make_spot()).items():
             print(f"{k:24s} oracle-vs-reference rel err {v:.2e}")
     else:
         main()

@@ -1,10 +1,9 @@
 """CPU: the oracle restatement against the committed golden vectors (outputs of the
-UNMODIFIED reference, tests/golden/, made by oracle/make_golden.py) and -- when
-/root/reference is present -- against the live reference."""
+UNMODIFIED reference, tests/golden/, made by oracle/make_golden.py)."""
 import numpy as np
 import pytest
 
-from oracle import dsp_oracle as O, detect_oracle as D, ref_loader
+from oracle import dsp_oracle as O, detect_oracle as D
 from conftest import rel_err
 
 DX = 2.0419046878814697
@@ -126,21 +125,23 @@ def test_sliding_dft_recursion_numerics(n_fft, hop, b0, b1):
     assert np.abs(O.stft_sliding_band(y, n_fft, hop, b0, b1, dtype=np.float64) - ref[b0:b1 + 1]).max() / ref.max() <= 1e-12
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present (GPU box)")
-def test_oracle_against_live_reference():
-    dsp, detect = ref_loader.load()
+def test_oracle_against_live_reference(golden):
+    """Spot check on seeded white noise against the reference's outputs for the same input (tests/golden/spot.npz;
+    every third row of the 2-D outputs is stored)."""
+    g = golden("spot")
     rng = np.random.default_rng(5)
     nx, ns = 36, 200
     x = rng.standard_normal((nx, ns))
+    assert abs(float(np.sum(x)) - float(g["a_x_checksum"])) <= 1e-9
     sel = [0, nx, 1]
-    m = dsp.fk_filter_design((nx, ns), sel, DX, FS)
+    m = g["a_mask"]
     assert np.array_equal(m, O.fk_filter_design((nx, ns), sel, DX, FS))
-    assert rel_err(O.fk_filter_filt(x.copy(), m, True), dsp.fk_filter_filt(x.copy(), m, True))[0] <= 1e-13
-    h = np.asarray(dsp.hybrid_ninf_filter_design((nx, ns), sel, DX, FS))
-    assert np.max(np.abs(h - O.hybrid_ninf_filter_design((nx, ns), sel, DX, FS))) <= 1e-13
-    assert rel_err(O.bp_filt(x, FS, 14, 30), dsp.bp_filt(x, FS, 14, 30))[0] <= 1e-13
-    tpl = detect.gen_template_fincall(np.arange(ns) / FS, FS, 17.8, 28.8, 0.68)
-    assert rel_err(D.compute_cross_correlogram(x, tpl), detect.compute_cross_correlogram(x, tpl))[0] <= 1e-13
+    assert rel_err(O.fk_filter_filt(x.copy(), m, True)[::3], g["a_fk_rows"])[0] <= 1e-13
+    assert np.max(np.abs(g["a_ninf"] - O.hybrid_ninf_filter_design((nx, ns), sel, DX, FS))) <= 1e-13
+    assert rel_err(O.bp_filt(x, FS, 14, 30)[::3], g["a_bp_rows"])[0] <= 1e-13
+    tpl = g["a_tpl"]
+    assert np.array_equal(tpl, D.gen_template_fincall(np.arange(ns) / FS, FS, 17.8, 28.8, 0.68))
+    assert rel_err(D.compute_cross_correlogram(x, tpl)[::3], g["a_xc_rows"])[0] <= 1e-13
 
 
 def test_picks_and_raw2strain_match_golden(golden):
@@ -208,15 +209,17 @@ def test_torch_second_oracle_pinned_to_numpy_oracle():
         assert rel_err(O.fk_filter_filt(x, mo, workers=2), O.fk_filter_filt(x, mo))[0] <= 1e-13     # bench's threaded CPU arm
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present (GPU box)")
-def test_round2_oracle_against_live_reference():
-    dsp, detect = ref_loader.load()
-    imp = ref_loader.load_improcess()
+def test_round2_oracle_against_live_reference(golden):
+    """Spot check of the spectral view and the image-detector helpers against the reference's outputs for the same
+    seeded input (tests/golden/spot.npz; the reference's Gabor `down` kernel is flipud(up))."""
     from oracle import improcess_oracle as IO
+    g = golden("spot")
     rng = np.random.default_rng(8)
     x = rng.standard_normal((30, 500))
-    assert rel_err(O.get_fx(x, 256), dsp.get_fx(x, 256))[0] <= 1e-14
-    assert rel_err(IO.trace2image(x), imp.trace2image(x))[0] <= 1e-13
-    assert rel_err(IO.binning(imp.trace2image(x), 0.1, 0.1), imp.binning(imp.trace2image(x), 0.1, 0.1))[0] <= 1e-13
-    up, down = imp.gabor_filt_design(40.0)
-    assert np.array_equal(up, IO.gabor_filt_design(40.0)[0]) and np.array_equal(down, IO.gabor_filt_design(40.0)[1])
+    assert abs(float(np.sum(x)) - float(g["b_x_checksum"])) <= 1e-9
+    assert rel_err(O.get_fx(x, 256)[::3], g["b_fx_rows"])[0] <= 1e-14
+    image = IO.trace2image(x)
+    assert rel_err(image[::3], g["b_img_rows"])[0] <= 1e-13
+    assert rel_err(IO.binning(image, 0.1, 0.1), g["b_bin"])[0] <= 1e-13
+    up, down = IO.gabor_filt_design(40.0)
+    assert np.array_equal(up, g["b_up"]) and np.array_equal(down, np.flipud(g["b_up"]))
